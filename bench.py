@@ -20,6 +20,11 @@
 /root/reference/src/*.cu) through the reference's own functions on the same workload.  The
 reference has no CPU implementation (SURVEY.md fact 8), so its own path IS a GPU path; the CPU
 figure (`cpu_baseline`, kind "port") is the oracle's OpenMP restatement on the host cores.
+
+--dump-outputs DIR (native path, rank 0) writes what the last timed step handed its caller, the frame's fp32 depth map and
+its 8-bit depth map, as DIR/depth.npy and DIR/depth_u8.npy in float32.  The inputs are seeded, so two builds run with the
+same arguments can be compared output for output.  Where both planes together exceed 64 MB (4K and up), both keep the same
+fixed, seeded sample of pixels; DIR/pixel_index.npy (float64) holds their row-major indices.
 """
 import argparse
 import json
@@ -41,6 +46,20 @@ WORKLOADS = {"8k": (4320, 7680, 1004), "4k": (2160, 3840, 1003), "1080p": (1080,
 # 93.5 MB read + 37.9 MB written); workloads without a capture report null
 NCU_TRAFFIC_BYTES_PER_LAUNCH = {"4k": 131.5e6}
 BYTES_PER_PIXEL_SWEEP = 17.0     # SURVEY.md section 8(d): x_k 4 + x_{k-1} 4 + x_{k+1} 4 + 4 link indices 4 + mask 1
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(outdir, planes):
+    """planes: [(name, 2-D array)] of one shape -> outdir/<name>.npy in float32, sampled as the module docstring says."""
+    os.makedirs(outdir, exist_ok=True)
+    n = planes[0][1].size
+    if 4 * n * len(planes) > DUMP_BYTES:
+        keep = (DUMP_BYTES - (1 << 16)) // (4 * len(planes) + 8)           # float32 per plane + one float64 index, headers aside
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        np.save(os.path.join(outdir, "pixel_index.npy"), idx.astype(np.float64))
+        planes = [(name, a.reshape(-1)[idx]) for name, a in planes]
+    for name, a in planes:
+        np.save(os.path.join(outdir, name + ".npy"), a.astype(np.float32))
 
 
 def peaks():
@@ -300,6 +319,10 @@ def run_native(args, dist, rank, world, local):
         barrier(dist)
         launches = ctx.launch_count - launches0
         ms_dev = max_over_ranks(dist, ev0.elapsed_time(ev1) / args.steps)
+        if args.dump_outputs and rank == 0:
+            # copied now: every later frame starts its coarsest level from this one's depth (main.cpp:257)
+            dumped = [("depth", ctx.frame_plane(ctx.PLANE_DEPTH, 0).cpu().numpy()),
+                      ("depth_u8", ctx.frame_plane(ctx.PLANE_DEPTH_U8, 0).cpu().numpy())]
         lvl_ms = [ctx.level_sweep_ms(l) for l in range(ctx.levels)]
         # level 0 of the same device-resident frame once more, one frame at a time, for the roofline's launch average (the level
         # events can only be read between frames)
@@ -418,6 +441,8 @@ def run_native(args, dist, rank, world, local):
         "clocks": clocks,
     }
     ctx.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
     return line
 
 
@@ -616,7 +641,12 @@ def main():
     ap.add_argument("--no-strips", action="store_true", help="skip the configs[4] record (16384^2 row strips)")
     ap.add_argument("--strips-size", type=int, default=16384, help="side of the configs[4] image")
     ap.add_argument("--seed-offset", type=int, default=0, help="extra offset on the synthetic image seed (diagnostics)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's depth maps to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs covers the native path")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE line, the JSON result: anything libraries print there meanwhile (NCCL's version banner
     # under NCCL_DEBUG=VERSION, for one) is sent to stderr instead

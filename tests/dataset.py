@@ -1,21 +1,20 @@
 """The reference's 12 dataset pairs as test fixtures (BASELINE configs[0]).
 
-tests/golden/dataset_pack.npz holds, per pair, the JPEG file's bytes and the annotation read as gray
-(what main.cpp reads: src/main.cpp:93 imread colour, :160-162 imread gray); it is written by
-tests/golden/make_golden_inputs.py in the container that has /root/reference, so nothing here touches that tree.
+tests/golden/dataset/<name>.npz holds, per pair, the JPEG file's bytes ("jpg") and the annotation read as gray ("ann"; what
+main.cpp reads: src/main.cpp:93 imread colour, :160-162 imread gray); written by tests/golden/make_golden_inputs.py --pack
+from the reference's dataset directory, so that the tests need nothing outside this repository.
 """
 import os
 
 import numpy as np
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-PACK = os.path.join(GOLD, "dataset_pack.npz")
+PAIRS = os.path.join(GOLD, "dataset")
 NAMES = ["arara", "archespark", "dog", "flower", "heidelberg", "hills", "pigs", "rock", "straw", "streetart", "vintagegirl", "womanparasol"]
-_pack = None
 
 
 def have_pack():
-    return os.path.exists(PACK)
+    return all(os.path.exists(os.path.join(PAIRS, name + ".npz")) for name in NAMES)
 
 
 def annotation_to_planes(bgr, ann):
@@ -28,12 +27,10 @@ def annotation_to_planes(bgr, ann):
 
 def load_pair(name):
     """-> (bgr, scribble, edited, annotation) of one dataset pair, decoded with the same cv2 the rest of the tests use."""
-    global _pack
     import cv2
-    if _pack is None:
-        _pack = np.load(PACK)
-    bgr = cv2.imdecode(_pack[name + "_jpg"], cv2.IMREAD_COLOR)
-    ann = _pack[name + "_ann"]
+    z = np.load(os.path.join(PAIRS, name + ".npz"))
+    bgr = cv2.imdecode(z["jpg"], cv2.IMREAD_COLOR)
+    ann = z["ann"]
     assert bgr is not None and bgr.shape[:2] == ann.shape
     scribble, edited = annotation_to_planes(bgr, ann)
     return bgr, scribble, edited, ann

@@ -126,7 +126,7 @@ def weights_case(api, libref, rows, cols, seed, levels, level):
 def dataset_goldens(api):
     """All 12 dataset pairs (BASELINE configs[0]) through the reference's own kernels, native resolution, 1000 sweeps at the
     coarsest level: per-level sha256 of the fp32 outputs, sha of the u8 map, and the same for a second frame with one more
-    stroke (state carried over).  Hashes only -- the inputs are in tests/golden/dataset_pack.npz."""
+    stroke (state carried over).  Hashes only -- the inputs are in tests/golden/dataset/."""
     import json
     from tests import dataset
     out = {}

@@ -24,21 +24,20 @@ def main(names):
 
 
 def pack_all():
-    """All 12 pairs in one file: the JPEG bytes as they are (decoded by cv2 at test time, like main.cpp's imread) and the
-    annotation as the gray plane main.cpp reads (3.3 MB instead of 12 x ~1 MB of decoded pixels)."""
+    """All 12 pairs, one file each under tests/golden/dataset/ (0.1 - 0.45 MB): the JPEG bytes as they are (decoded by cv2 at
+    test time, like main.cpp's imread) and the annotation as the gray plane main.cpp reads."""
     import glob
-    pack = {}
+    outdir = os.path.join(ROOT, "tests", "golden", "dataset")
+    os.makedirs(outdir, exist_ok=True)
     for f in sorted(glob.glob(os.path.join(REF, "images", "*.jpg"))):
         name = os.path.basename(f)[:-4]
         raw = np.fromfile(f, np.uint8)
         assert np.array_equal(cv2.imread(f), cv2.imdecode(raw, cv2.IMREAD_COLOR))
         ann = cv2.imread(os.path.join(REF, "annotations", name + ".png"), 0)
         assert ann is not None
-        pack[name.lower() + "_jpg"] = raw
-        pack[name.lower() + "_ann"] = ann
-    out = os.path.join(ROOT, "tests", "golden", "dataset_pack.npz")
-    np.savez_compressed(out, **pack)
-    print(out, len(pack) // 2, "pairs", os.path.getsize(out))
+        out = os.path.join(outdir, name.lower() + ".npz")
+        np.savez_compressed(out, jpg=raw, ann=ann)
+        print(out, os.path.getsize(out))
 
 
 if __name__ == "__main__":

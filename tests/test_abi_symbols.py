@@ -39,15 +39,14 @@ def test_reference_headers_declare_the_same_ten_functions():
 
 
 def test_libref_exports_identical_mangled_names():
-    """When the reference kernels were compiled (oracle/_ref), their symbols must be the ones we ship."""
-    from oracle import binding as ob
+    """The mangled names the reference's own library exports (tests/golden/ref_ab.json) are the ones we bind and ship."""
     from realtimedepthdiffusion_b200 import _native
-    if not os.path.exists(ob.LIBREF):
-        import pytest
-        pytest.skip("oracle/_ref/libref.so not built")
-    out = os.popen("nm -D --defined-only %s" % ob.LIBREF).read()
-    for sym in _native.SHIM_SYMBOLS.values():
-        assert sym in out, sym
+    from tests.harness import reference_golden
+    ref_symbols = reference_golden("symbols")
+    assert sorted(_native.SHIM_SYMBOLS.values()) == sorted(ref_symbols)
+    out = os.popen("nm -D --defined-only %s" % _native.LIB_PATH).read()
+    for sym in ref_symbols:
+        assert re.search(r"\b%s\b" % sym, out), sym
 
 
 def test_host_helpers_without_a_gpu():

@@ -1,7 +1,6 @@
 """The drop-in claim from the reference's own language: tests/cpp/main_like.cpp is written only against the three
 reference-named headers (like main.cpp).  It must compile and link against librtdd.so without source changes (CPU test)
-and, on the GPU box, produce bit-identical output whether it is linked against librtdd.so or against the reference's
-own kernels (oracle/_ref/libref.so)."""
+and, on a GPU, produce the output it produced when linked against the reference's own kernels (tests/golden/ref_ab.json)."""
 import os
 import re
 import subprocess
@@ -32,19 +31,22 @@ def test_main_like_links_against_librtdd_unchanged():
         assert re.search(r"\b%s\(" % fn, undefined), fn        # resolved at load time from librtdd.so
 
 
+def main_like_line(tag, libdir, lib, rows, cols, iters):
+    """The checksum line main_like prints when linked against lib<lib>.so in `libdir`."""
+    exe = build(tag, libdir, lib)
+    r = subprocess.run([exe, str(rows), str(cols), str(iters)], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=280)
+    assert r.returncode == 0, r.stdout
+    return [ln for ln in r.stdout.splitlines() if ln.startswith("levels")][-1]
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("rows,cols,iters", [(203, 317, 100), (624, 672, 1000)])
 def test_main_like_same_output_with_reference_kernels_and_with_librtdd(rows, cols, iters):
-    refdir = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.exists(os.path.join(refdir, "libref.so")):
-        pytest.skip("oracle/_ref/libref.so not built")
-    outs = {}
-    for tag, libdir, lib in (("rtdd", os.path.join(ROOT, "realtimedepthdiffusion_b200", "lib"), "rtdd"), ("ref", refdir, "ref")):
-        exe = build(tag, libdir, lib)
-        r = subprocess.run([exe, str(rows), str(cols), str(iters)], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=280)
-        assert r.returncode == 0, r.stdout
-        outs[tag] = [ln for ln in r.stdout.splitlines() if ln.startswith("levels")][-1]
-    assert outs["rtdd"] == outs["ref"], outs
+    """Linked against librtdd.so, main_like prints the line it printed when linked against the reference's own kernels
+    (tests/golden/ref_ab.json)."""
+    from tests.harness import reference_golden
+    want = reference_golden("main_like")["%dx%dx%d" % (rows, cols, iters)]
+    assert main_like_line("rtdd", os.path.join(ROOT, "realtimedepthdiffusion_b200", "lib"), "rtdd", rows, cols, iters) == want
 
 
 # ---- the multi-GPU entry points from a C++ host ------------------------------------------------------------------------------

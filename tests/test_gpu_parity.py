@@ -1,6 +1,6 @@
-"""GPU parity tests (run on the B200 box): librtdd.so through its C ABI and through the
-reference-named C++ shims, against (1) the CPU oracle, (2) the reference's own kernels
-(oracle/_ref/libref.so) in the same process, (3) the committed golden vectors.
+"""GPU parity tests (run on a B200): librtdd.so through its C ABI and through the
+reference-named C++ shims, against (1) the CPU oracle, (2) the results of the reference's own
+kernels on the same calls, (3) the committed golden vectors.
 
 Bars: solver floats BIT-EXACT (stronger than north_star's 1e-4 relative L-inf, which the chained
 pyramid needs anyway -- SURVEY.md fact 6); u8 outputs identical, except haze against the CPU
@@ -16,7 +16,7 @@ import torch
 
 from oracle import binding as ob
 from realtimedepthdiffusion_b200 import synth
-from tests.harness import MainLoop, pitch, ptr, to_dev, to_host
+from tests.harness import MainLoop, pitch, ptr, reference_golden, to_dev, to_host
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -481,63 +481,59 @@ def test_effects_vs_oracle(rtdd, rows, cols):
     ctx.close()
 
 
-# ---- A/B against the reference's own kernels in the same process --------------------------------
+# ---- A/B against the reference's own kernels (their results stored under tests/golden/) --------------------------------
 
-def have_ref():
-    return os.path.exists(ob.LIBREF)
-
-
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref/libref.so not built")
 @pytest.mark.parametrize("name", ["synth_tiny", "synth_odd", "dog", "womanparasol"])
 def test_main_loop_ab_reference_vs_shims(name):
-    """The same restated main.cpp loop, once over the reference's functions and once over ours."""
+    """The restated main.cpp loop over our reference-named functions, two frames (the second with one more stroke, state carried
+    over), against what the same loop computed over the reference's own kernels (tests/golden/ref_solver_<name>.npz)."""
     from realtimedepthdiffusion_b200 import _native
     from tests.test_oracle_cpu import _load_case
+    z = np.load(os.path.join(GOLD, "ref_solver_%s.npz" % name))
     bgr, scribble, edited = _load_case(name)
     iters = {"dog": 1000, "womanparasol": 1000, "synth_odd": 200, "synth_tiny": 60}[name]
-    res = {}
-    for tag, api in (("ref", ob.ref_api()), ("new", _native.shims)):
-        loop = MainLoop(api, bgr)
-        u8 = loop.frame(scribble, edited, iters, keep_levels=True)
-        ev = synth.brush_events(loop.rows, loop.cols, 99, 1, 6)
-        s2, e2 = synth.paint_events(bgr, ev, scribble.copy(), edited.copy())
-        u8b = loop.frame(s2, e2, iters)
-        res[tag] = (u8, {l: d["out"] for l, d in loop.per_level.items()}, u8b, loop.depth_float)
-        loop.close()
-    for l in res["ref"][1]:
-        a, b = res["ref"][1][l], res["new"][1][l]
-        assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), "level %d: max diff %g" % (l, np.abs(a - b).max())
-    assert np.array_equal(res["ref"][0], res["new"][0])
-    assert np.array_equal(res["ref"][2], res["new"][2])            # second frame (state carried over)
-    assert np.array_equal(res["ref"][3].view(np.uint32), res["new"][3].view(np.uint32))
+    assert int(z["max_iterations"]) == iters
+    loop = MainLoop(_native.shims, bgr)
+    u8 = loop.frame(scribble, edited, iters, keep_levels=True)
+    ev = synth.brush_events(loop.rows, loop.cols, 99, 1, 6)
+    s2, e2 = synth.paint_events(bgr, ev, scribble.copy(), edited.copy())
+    u8b = loop.frame(s2, e2, iters)
+    loop.close()
+    for l, d in loop.per_level.items():
+        assert sha(d["out"]) == str(z["out_sha_%d" % l]), "level %d" % l
+    assert np.array_equal(u8, z["depth_u8"])
+    assert np.array_equal(u8b, z["frame2_depth_u8"])            # second frame (state carried over)
+    assert sha(loop.depth_float) == str(z["frame2_out_sha_0"])
 
 
-@pytest.mark.skipif(not have_ref(), reason="oracle/_ref/libref.so not built")
-def test_effects_and_image_ops_ab_reference():
-    from realtimedepthdiffusion_b200 import _native
+def effects_and_paint(api):
+    """The three effects and two brush strokes through the ten reference-named functions of `api` on device planes:
+    {output: sha256 of its bytes}."""
     rows, cols = 203, 317
     bgr, gray, depth = effect_inputs(rows, cols, 33)
     o, g, d = to_dev(bgr, 3), to_dev(gray), to_dev(depth)
-    outs = {}
-    for tag, api in (("ref", ob.ref_api()), ("new", _native.shims)):
-        r = []
-        for name in ("GPUSimulateDesaturation", "GPUSimulateHaze", "GPUSimulateDefocus"):
-            out = to_dev(np.zeros_like(bgr), 3)
-            torch.cuda.synchronize()
-            if name == "GPUSimulateDesaturation":
-                api[name](ptr(o), pitch(o), ptr(g), pitch(g), ptr(d), pitch(d), ptr(out), pitch(out), rows, cols)
-            else:
-                api[name](ptr(o), pitch(o), ptr(d), pitch(d), ptr(out), pitch(out), rows, cols)
-            torch.cuda.synchronize()
-            r.append(to_host(out, 3))
-        e0, s0 = to_dev(bgr, 3), to_dev(np.zeros((rows, cols), np.uint8))
-        api["GPUPaintImage"](100, 50, 192, 9, ptr(e0), pitch(e0), ptr(s0), pitch(s0), rows, cols)
-        api["GPUPaintImage"](2, 200, 64, 14, ptr(e0), pitch(e0), ptr(s0), pitch(s0), rows, cols)
+    r = {}
+    for name in ("GPUSimulateDesaturation", "GPUSimulateHaze", "GPUSimulateDefocus"):
+        out = to_dev(np.zeros_like(bgr), 3)
         torch.cuda.synchronize()
-        r += [to_host(e0, 3), to_host(s0)]
-        outs[tag] = r
-    for a, b in zip(outs["ref"], outs["new"]):
-        assert np.array_equal(a, b)
+        if name == "GPUSimulateDesaturation":
+            api[name](ptr(o), pitch(o), ptr(g), pitch(g), ptr(d), pitch(d), ptr(out), pitch(out), rows, cols)
+        else:
+            api[name](ptr(o), pitch(o), ptr(d), pitch(d), ptr(out), pitch(out), rows, cols)
+        torch.cuda.synchronize()
+        r[name] = sha(to_host(out, 3))
+    e0, s0 = to_dev(bgr, 3), to_dev(np.zeros((rows, cols), np.uint8))
+    api["GPUPaintImage"](100, 50, 192, 9, ptr(e0), pitch(e0), ptr(s0), pitch(s0), rows, cols)
+    api["GPUPaintImage"](2, 200, 64, 14, ptr(e0), pitch(e0), ptr(s0), pitch(s0), rows, cols)
+    torch.cuda.synchronize()
+    r["GPUPaintImage edited"] = sha(to_host(e0, 3))
+    r["GPUPaintImage scribble"] = sha(to_host(s0))
+    return r
+
+
+def test_effects_and_image_ops_ab_reference():
+    from realtimedepthdiffusion_b200 import _native
+    assert effects_and_paint(_native.shims) == reference_golden("effects_and_paint_203x317")
 
 
 # ---- whole-frame entry point -------------------------------------------------------------------

@@ -1,8 +1,8 @@
-"""GPU parity at the sizes the bench measures (VERDICT r01, Weak #1): the whole frame against the reference's OWN kernels
-(oracle/_ref/libref.so) at 1920x1080 (BASELINE configs[1], 32-event stroke replay with carried state) and 3840x2160
-(configs[2] incl. the three depth effects, defocus box up to 110), the finest level of a 16384 x 16384 image (configs[4]),
-the persistent TMA kernel's region loop forced through many trips per CTA against the CPU oracle, and all 12 dataset pairs
-(configs[0]) against hashes recorded from the reference.  Bar: bit-exact floats, identical bytes."""
+"""GPU parity at the sizes the bench measures (VERDICT r01, Weak #1): the whole frame against what the reference's OWN kernels
+computed (hashes in tests/golden/ref_ab.json) at 1920x1080 (BASELINE configs[1], 32-event stroke replay with carried state) and
+3840x2160 (configs[2] incl. the three depth effects, defocus box up to 110), the finest level of a 16384 x 16384 image
+(configs[4]), the persistent TMA kernel's region loop forced through many trips per CTA against the CPU oracle, and all 12
+dataset pairs (configs[0]) against hashes recorded from the reference.  Bar: bit-exact floats, identical bytes."""
 import hashlib
 import json
 import os
@@ -16,12 +16,11 @@ import torch
 from oracle import binding as ob
 from realtimedepthdiffusion_b200 import synth
 from tests import dataset
-from tests.harness import MainLoop, pitch, ptr, to_dev, to_host
+from tests.harness import MainLoop, pitch, ptr, reference_golden, to_dev, to_host
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-need_ref = pytest.mark.skipif(not os.path.exists(ob.LIBREF), reason="oracle/_ref/libref.so not built")
 
 
 def sha(a):
@@ -32,10 +31,6 @@ def sha(a):
 def rtdd():
     import realtimedepthdiffusion_b200 as pkg
     return pkg
-
-
-def bits_equal(a, b):
-    return torch.equal(a.contiguous().view(torch.int32), b.contiguous().view(torch.int32))
 
 
 # ---- the persistent kernel's region loop, many trips per CTA, against the oracle ----------------------------------------
@@ -75,51 +70,57 @@ def test_persistent_region_loop_many_trips_vs_oracle(rtdd, rows, cols, cap, mode
 
 
 # ---- whole frames against the reference's own kernels at the benchmarked sizes -----------------------------------------
+# The reference's results are stored as hashes in tests/golden/ref_ab.json; the functions below compute both sides: over the
+# reference's own library when tests/golden/gen_golden_ab.py records them, over librtdd.so's shims in the tests.
 
-def _ab_frames(bgr, frames, effects=False):
-    """The restated main.cpp loop over the reference's functions and over ours: per-level floats and u8 maps of every frame
-    (kept on the host as hashes), optionally followed by the three effects on the last frame's depth."""
-    from realtimedepthdiffusion_b200 import _native
-    out = {}
-    for tag, api in (("ref", ob.ref_api()), ("new", _native.shims)):
-        loop = MainLoop(api, bgr)
-        rec = []
-        for scribble, edited in frames:
-            u8 = loop.frame(scribble, edited, 1000, keep_levels=True)
-            rec.append(([sha(loop.per_level[l]["out"]) for l in range(loop.levels)], sha(u8), sha(loop.depth_float)))
-        eff = []
-        if effects:
-            rows, cols = loop.rows, loop.cols
-            for name in ("GPUSimulateDesaturation", "GPUSimulateHaze", "GPUSimulateDefocus"):
-                o = to_dev(np.zeros_like(bgr), 3)
-                torch.cuda.synchronize()
-                if name == "GPUSimulateDesaturation":
-                    api[name](ptr(loop.orig), pitch(loop.orig), ptr(loop.gray[0]), pitch(loop.gray[0]), ptr(loop.depth[0]), pitch(loop.depth[0]),
-                              ptr(o), pitch(o), rows, cols)
-                else:
-                    api[name](ptr(loop.orig), pitch(loop.orig), ptr(loop.depth[0]), pitch(loop.depth[0]), ptr(o), pitch(o), rows, cols)
-                torch.cuda.synchronize()
-                eff.append(sha(to_host(o, 3)))
-        out[tag] = (rec, eff, loop.depth_float.copy())
-        loop.close()
-    return out
+def main_loop_hashes(api, bgr, frames, effects=False):
+    """The restated main.cpp loop over the ten reference-named functions of `api`: per-level floats, u8 map and fp32 map of
+    every frame as hashes, optionally followed by the three effects on the last frame's depth."""
+    loop = MainLoop(api, bgr)
+    rec = []
+    for scribble, edited in frames:
+        u8 = loop.frame(scribble, edited, 1000, keep_levels=True)
+        rec.append([[sha(loop.per_level[l]["out"]) for l in range(loop.levels)], sha(u8), sha(loop.depth_float)])
+    eff = []
+    if effects:
+        rows, cols = loop.rows, loop.cols
+        for name in ("GPUSimulateDesaturation", "GPUSimulateHaze", "GPUSimulateDefocus"):
+            o = to_dev(np.zeros_like(bgr), 3)
+            torch.cuda.synchronize()
+            if name == "GPUSimulateDesaturation":
+                api[name](ptr(loop.orig), pitch(loop.orig), ptr(loop.gray[0]), pitch(loop.gray[0]), ptr(loop.depth[0]), pitch(loop.depth[0]),
+                          ptr(o), pitch(o), rows, cols)
+            else:
+                api[name](ptr(loop.orig), pitch(loop.orig), ptr(loop.depth[0]), pitch(loop.depth[0]), ptr(o), pitch(o), rows, cols)
+            torch.cuda.synchronize()
+            eff.append(sha(to_host(o, 3)))
+    loop.close()
+    return {"frames": rec, "effects": eff}
 
 
-@need_ref
-def test_1080p_stroke_replay_ab_reference(rtdd):
-    """BASELINE configs[1]: 1920x1080, seed 1002, 32 brush events, one full frame per event, state carried between frames
-    exactly like main.cpp (the coarsest depth plane persists).  Also: the whole-frame entry point with device-side painting
-    (rtdd_frame_paint + rtdd_frame_solve) reproduces the reference's last frame."""
+def stroke_replay_1080p():
+    """BASELINE configs[1]: 1920x1080, seed 1002, 32 brush events (4 strokes x 8), the annotation planes after each event."""
     rows, cols = 1080, 1920
     bgr = synth.synth_image(rows, cols, 1002)
-    events = synth.brush_events(rows, cols, 1002, 4, 8)           # 4 strokes x 8 events = 32
-    assert len(events) == 32
+    events = synth.brush_events(rows, cols, 1002, 4, 8)
     frames, s, e = [], np.zeros((rows, cols), np.uint8), bgr.copy()
     for ev in events:
         s, e = synth.paint_events(bgr, [ev], s, e)
         frames.append((s.copy(), e.copy()))
-    out = _ab_frames(bgr, frames)
-    for k, (a, b) in enumerate(zip(out["ref"][0], out["new"][0])):
+    return bgr, events, frames
+
+
+def test_1080p_stroke_replay_ab_reference(rtdd):
+    """BASELINE configs[1]: 1920x1080, seed 1002, 32 brush events, one full frame per event, state carried between frames
+    exactly like main.cpp (the coarsest depth plane persists).  Also: the whole-frame entry point with device-side painting
+    (rtdd_frame_paint + rtdd_frame_solve) reproduces the reference's last frame."""
+    from realtimedepthdiffusion_b200 import _native
+    want = reference_golden("stroke_replay_1080p")
+    bgr, events, frames = stroke_replay_1080p()
+    rows, cols = bgr.shape[:2]
+    assert len(events) == 32 == len(want["frames"])
+    got = main_loop_hashes(_native.shims, bgr, frames)
+    for k, (a, b) in enumerate(zip(want["frames"], got["frames"])):
         assert a == b, "frame %d differs from the reference's kernels" % k
     ctx = rtdd.DepthDiffusion(rows, cols)
     ctx.frame_set_image(bgr)
@@ -129,33 +130,33 @@ def test_1080p_stroke_replay_ab_reference(rtdd):
         ctx.frame_paint(*ev)
         ctx.frame_solve(1000)
     ctx.sync()
-    got = ctx.frame_plane(ctx.PLANE_DEPTH, 0).cpu().numpy()
-    assert np.array_equal(got.view(np.uint32), out["ref"][2].view(np.uint32))
-    assert sha(ctx.frame_plane(ctx.PLANE_DEPTH_U8, 0).cpu().numpy()) == out["ref"][0][-1][1]
+    assert sha(ctx.frame_plane(ctx.PLANE_DEPTH, 0).cpu().numpy()) == want["frames"][-1][2]
+    assert sha(ctx.frame_plane(ctx.PLANE_DEPTH_U8, 0).cpu().numpy()) == want["frames"][-1][1]
     ctx.close()
 
 
-@need_ref
 def test_4k_frame_and_effects_ab_reference(rtdd):
     """BASELINE configs[2] -- the bench workload itself (3840x2160, seed 1003, ~10 % scribbles, 6 levels, 1968 sweeps) and the
     three effects on the solved depth (defocus box side up to 110: the exact summed-area path at its largest measured size),
     against the reference's own kernels; then the whole-frame entry points (3-plane and single-plane annotation upload)."""
+    from realtimedepthdiffusion_b200 import _native
+    want = reference_golden("frame_4k")
     rows, cols = 2160, 3840
     bgr, scribble, edited = synth.synth_case(rows, cols, 1003)
-    out = _ab_frames(bgr, [(scribble, edited)], effects=True)
-    assert out["ref"][0] == out["new"][0], "per-level floats / u8 map differ from the reference's kernels"
-    assert out["ref"][1] == out["new"][1], "effects differ from the reference's kernels"
-    want_u8, want_f = out["ref"][0][0][1], out["ref"][2]
+    got = main_loop_hashes(_native.shims, bgr, [(scribble, edited)], effects=True)
+    assert got["frames"] == want["frames"], "per-level floats / u8 map differ from the reference's kernels"
+    assert got["effects"] == want["effects"], "effects differ from the reference's kernels"
+    want_u8, want_f = want["frames"][0][1], want["frames"][0][2]
     ctx = rtdd.DepthDiffusion(rows, cols)
     ctx.frame_set_image(bgr)
     u8 = ctx.frame_solve_host(scribble, edited, 1000, np.zeros((rows, cols), np.uint8)).numpy()
     assert sha(u8) == want_u8
-    assert np.array_equal(ctx.frame_plane(ctx.PLANE_DEPTH, 0).cpu().numpy().view(np.uint32), want_f.view(np.uint32))
+    assert sha(ctx.frame_plane(ctx.PLANE_DEPTH, 0).cpu().numpy()) == want_f
     # the frame path's effects (cached summed-area table) on the same depth
     outs = [to_dev(np.zeros_like(bgr), 3) for _ in range(3)]
     ctx.frame_effects(*outs)
     ctx.sync()
-    assert [sha(to_host(o, 3)) for o in outs] == out["ref"][1]
+    assert [sha(to_host(o, 3)) for o in outs] == want["effects"]
     # single-plane annotation upload: same frame
     ctx2 = rtdd.DepthDiffusion(rows, cols)
     ctx2.frame_set_image(bgr)
@@ -200,32 +201,39 @@ def device_level(rows, cols, seed, dev="cuda"):
     return gray, depth, scribble
 
 
-@need_ref
+def dev_sha(t):
+    return sha(t.cpu().numpy())
+
+
+def finest_level(api, size, sweeps):
+    """Level 0 of a size x size device-generated level (one level allocated: 6.4 GB of scratch at 16384), `sweeps` sweeps of
+    `api`'s GPUMatrixFreeSolver -> (gray, depth guess, scribble, solved depth)."""
+    from realtimedepthdiffusion_b200.api import pitched_empty
+    rows = cols = size
+    gray, depth, scribble = device_level(rows, cols, 1005)
+    d = pitched_empty(rows, cols, torch.float32, "cuda")
+    d.copy_(depth)
+    torch.cuda.synchronize()
+    api["GPUAllocateDeviceMemory"](rows, cols, 1)
+    api["GPULoadWeights"](0.4)
+    # level 0 of a 1-level pyramid is the ungated coarsest level; the gated variant is covered by the 4K frame
+    api["GPUMatrixFreeSolver"](ptr(d), pitch(d), ptr(scribble), pitch(scribble), ptr(gray), pitch(gray), rows, cols, 0.4, sweeps, 1e-5, 0)
+    torch.cuda.synchronize()
+    api["GPUFreeDeviceMemory"](1)
+    return gray, depth, scribble, d
+
+
 @pytest.mark.parametrize("size,sweeps", [(16384, 64)])
 def test_16k_finest_level_ab_reference(rtdd, size, sweeps):
     """BASELINE configs[4], measurement (i): level 0 of a 16384 x 16384 image, 64 sweeps, against the reference's
-    GPUMatrixFreeSolver on the same device planes (one level allocated on each side: 6.4 GB + 5.1 GB of scratch)."""
+    GPUMatrixFreeSolver on the same device planes."""
     from realtimedepthdiffusion_b200 import _native
-    rows = cols = size
-    gray, depth, scribble = device_level(rows, cols, 1005)
-    torch.cuda.synchronize()
-    results = []
-    for api in (ob.ref_api(), _native.shims):
-        from realtimedepthdiffusion_b200.api import pitched_empty
-        d = pitched_empty(rows, cols, torch.float32, "cuda")
-        d.copy_(depth)
-        torch.cuda.synchronize()
-        api["GPUAllocateDeviceMemory"](rows, cols, 1)
-        api["GPULoadWeights"](0.4)
-        # level 0 of a 1-level pyramid is the ungated coarsest level; the gated variant is covered by the 4K frame
-        api["GPUMatrixFreeSolver"](ptr(d), pitch(d), ptr(scribble), pitch(scribble), ptr(gray), pitch(gray), rows, cols, 0.4, sweeps, 1e-5, 0)
-        torch.cuda.synchronize()
-        api["GPUFreeDeviceMemory"](1)
-        results.append(d)
-    assert bits_equal(results[0], results[1])
+    want = reference_golden("level0_%d_x%d" % (size, sweeps))
+    gray, depth, scribble, got = finest_level(_native.shims, size, sweeps)
+    assert [dev_sha(gray), dev_sha(depth), dev_sha(scribble)] == want["inputs"], "the device-generated inputs changed"
+    assert dev_sha(got) == want["depth"]
     m = scribble == 255
-    assert torch.equal(results[1][m], depth[m])                  # Dirichlet pixels untouched
-    del results
+    assert torch.equal(got[m], depth[m])                         # Dirichlet pixels untouched
 
 
 # ---- DepthEffect on row strips (one GPU plays every rank in turn) and the huge-box fallback ------------------------------------
@@ -259,12 +267,8 @@ def test_effects_on_row_strips_equal_the_whole_image(rtdd, rows, cols, nstrips):
     ctx.close()
 
 
-@need_ref
-def test_defocus_box_beyond_256_takes_the_raster_path_ab_reference(rtdd):
-    """K > 256 needs a diagonal beyond 10 240 pixels (ref: src/GPUDepthEffect.cu:42): 7400 x 7400 -> K = 261.  A box side above 256
-    makes the reference's fp32 sums inexact, so the exact summed-area table is not allowed there and the kernel replays the
-    reference's raster-order accumulation (effect_kernels.cu).  Mostly shallow depths keep the reference's own gather short."""
-    from realtimedepthdiffusion_b200 import _native
+def defocus_7400(api):
+    """GPUSimulateDefocus of `api` on a 7400 x 7400 device-generated image and depth -> (bgr, depth, out)."""
     from realtimedepthdiffusion_b200.api import pitched_empty
     rows = cols = 7400
     g = torch.Generator(device="cuda")
@@ -275,14 +279,22 @@ def test_defocus_box_beyond_256_takes_the_raster_path_ab_reference(rtdd):
     depth.copy_(torch.rand((rows, cols), generator=g, device="cuda") * 12.0)
     idx = torch.randint(0, rows * cols, (400,), generator=g, device="cuda")
     depth[idx // cols, idx % cols] = 252.0 + 3.0 * torch.rand(400, generator=g, device="cuda")      # a in 258 .. 261
-    outs = []
-    for api in (ob.ref_api(), _native.shims):
-        out = pitched_empty(rows, cols, torch.uint8, "cuda", channels=3, fill=0)
-        torch.cuda.synchronize()
-        api["GPUSimulateDefocus"](ptr(bgr), pitch(bgr), ptr(depth), pitch(depth), ptr(out), pitch(out), rows, cols)
-        torch.cuda.synchronize()
-        outs.append(out)
-    assert torch.equal(outs[0], outs[1])
+    out = pitched_empty(rows, cols, torch.uint8, "cuda", channels=3, fill=0)
+    torch.cuda.synchronize()
+    api["GPUSimulateDefocus"](ptr(bgr), pitch(bgr), ptr(depth), pitch(depth), ptr(out), pitch(out), rows, cols)
+    torch.cuda.synchronize()
+    return bgr, depth, out
+
+
+def test_defocus_box_beyond_256_takes_the_raster_path_ab_reference(rtdd):
+    """K > 256 needs a diagonal beyond 10 240 pixels (ref: src/GPUDepthEffect.cu:42): 7400 x 7400 -> K = 261.  A box side above 256
+    makes the reference's fp32 sums inexact, so the exact summed-area table is not allowed there and the kernel replays the
+    reference's raster-order accumulation (effect_kernels.cu).  Mostly shallow depths keep the reference's own gather short."""
+    from realtimedepthdiffusion_b200 import _native
+    want = reference_golden("defocus_7400")
+    bgr, depth, out = defocus_7400(_native.shims)
+    assert [dev_sha(bgr), dev_sha(depth)] == want["inputs"], "the device-generated inputs changed"
+    assert dev_sha(out) == want["out"]
     big = (depth.contiguous() * 261.0 / 255.0).int() > 256
     assert int(big.sum()) >= 300                                 # the raster path really ran
 

@@ -269,6 +269,16 @@ int rtdd_effects_rows(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, cons
                       const float *depth, size_t depthPitch, uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch,
                       uint8_t *defocus, size_t defocusPitch, int rows, int cols, int rowBegin, int rowEnd);
 
+/* Extension, no reference counterpart: depth-of-field refocus of a device image by a device depth plane (see DESIGN.md §7).
+ * Per pixel, with d' = depth clamped to [0, 255] (NaN -> 0): e = max(|d' - focusDepth| - depthOfField, 0),
+ * a = (int)((double)((float)aperture * e) / 255.0), h = a / 2; h = 0 copies the pixel, otherwise every channel is the floor of
+ * the exact mean of orig over [y-h, y+h) x [x-h, x+h) clipped to the image.  focusDepth in [0, 255]; depthOfField (the half-width
+ * of the sharp band, depth units) finite and >= 0; aperture (the largest box side, pixels) <= 4096, a negative one selects the
+ * reference defocus's K = (int)(0.025 x diagonal).  focusDepth = 0, depthOfField = 0, aperture = K gives rtdd_defocus's bytes
+ * for every depth <= 255 while K <= 257.  Builds the summed-area table of orig (4 launches) and refocuses (1). */
+int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                 uint8_t *out, size_t outPitch, int rows, int cols, float focusDepth, float depthOfField, int aperture);
+
 /* ---- pyramid ops either side of the path (SURVEY.md section 8f) ------------------- */
 
 /* cv::cvtColor(BGR2GRAY)                 ref: src/main.cpp:111,138 */
@@ -331,6 +341,12 @@ int rtdd_frame_solve_band(rtdd_ctx *ctx, int maxIterations, int rowBegin, int ro
  * caller-owned DEVICE planes (BGR u8, byte pitches; any of the three may be NULL).  The defocus summed-area table depends
  * on the image only and is built once per rtdd_frame_set_image, not once per call. */
 int rtdd_frame_effects(rtdd_ctx *ctx, uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch, uint8_t *defocus, size_t defocusPitch);
+/* rtdd_refocus on the frame context's own image and solved level-0 depth, with the cached summed-area table (shared with
+ * rtdd_frame_effects; built only when absent: 1 launch, else 5).
+ * focusX, focusY inside the image: focus = clamped depth under that pixel, read on the device (focusDepth ignored) -- a graph
+ * captured from this call follows every later solve;  focusX = focusY = -1: focus = focusDepth. */
+int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX, int focusY, float focusDepth,
+                       float depthOfField, int aperture);
 /* ref: src/main.cpp:46-62 -- brush stroke into the context's level-0 annotation planes */
 int rtdd_frame_paint(rtdd_ctx *ctx, int x, int y, int scribbleColor, int scribbleRadius);
 /* device pointers/pitches of the context-owned planes (for effects, tests, downloads) */

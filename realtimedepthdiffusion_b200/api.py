@@ -211,6 +211,14 @@ class DepthDiffusion:
         self._ck(lib.rtdd_effects_fused(self._h, _ptr(orig), _pitch(orig), _ptr(gray), _pitch(gray), _ptr(depth), _pitch(depth),
                                         _ptr(desat), _pitch(desat), _ptr(haze), _pitch(haze), _ptr(defocus), _pitch(defocus), rows, cols))
 
+    def refocus(self, orig, depth, out, focus_depth, depth_of_field=0.0, aperture=None):
+        """Extension (no reference counterpart): depth-of-field blur of `orig` by `depth` with the sharp band
+        [focus_depth - depth_of_field, focus_depth + depth_of_field] and a box of at most `aperture` pixels a side
+        (None = the reference defocus's K for the image size).  See rtdd_refocus in include/rtdd.h."""
+        rows, cols = depth.shape
+        self._ck(lib.rtdd_refocus(self._h, _ptr(orig), _pitch(orig), _ptr(depth), _pitch(depth), _ptr(out), _pitch(out), rows, cols,
+                                  float(focus_depth), float(depth_of_field), -1 if aperture is None else int(aperture)))
+
     # -- pyramid ops ---------------------------------------------------------------
     def bgr2gray(self, bgr, gray):
         rows, cols = gray.shape
@@ -295,6 +303,19 @@ class DepthDiffusion:
         """GPUSimulateDesaturation / Haze / Defocus on the frame's own image and solved depth (ref: src/main.cpp:190-230);
         outputs are device BGR planes, any may be None.  The defocus summed-area table is cached per image."""
         self._ck(lib.rtdd_frame_effects(self._h, _ptr(desat), _pitch(desat), _ptr(haze), _pitch(haze), _ptr(defocus), _pitch(defocus)))
+
+    def frame_refocus(self, out, focus_point=None, focus_depth=None, depth_of_field=0.0, aperture=None):
+        """refocus() of the frame's own image by its solved depth into the device BGR plane `out`, with the summed-area table
+        cached per image.  Give exactly one of focus_point = (x, y), whose depth is read on the GPU (no host round trip, so a
+        captured graph follows later solves), and focus_depth."""
+        if (focus_point is None) == (focus_depth is None):
+            raise ValueError("frame_refocus: give exactly one of focus_point and focus_depth")
+        if focus_point is None:
+            fx, fy, fd = -1, -1, float(focus_depth)
+        else:                 # NaN: a point of (-1, -1) is refused like any other point outside the image
+            fx, fy, fd = int(focus_point[0]), int(focus_point[1]), float("nan")
+        self._ck(lib.rtdd_frame_refocus(self._h, _ptr(out), _pitch(out), fx, fy, fd, float(depth_of_field),
+                                        -1 if aperture is None else int(aperture)))
 
     PLANE_DEPTH, PLANE_GRAY, PLANE_SCRIBBLE, PLANE_EDITED, PLANE_BGR, PLANE_DEPTH_U8 = range(6)
 

@@ -596,4 +596,90 @@ cudaError_t launch_defocus(cudaStream_t s, void *scratch, const uint8_t *orig, s
                                               defocus, defocusPitch, sat, aux, K, rows, cols, yBegin, yEnd, satRow0, satRows);
 }
 
+// ---------------------------------------------------------------------------
+// refocus (extension, no reference counterpart): box blur whose side grows with the distance of a pixel's depth from a focus
+// plane, over the same summed-area table as defocus.
+//   d' = clamp(d, 0, 255) (NaN -> 0); e = max(|d' - f| - w, 0); a = cvt.rzi.s32.f64((double)((float)A * e) / 255.0); h = a / 2;
+//   h == 0: copy; else out_c = floor(S_c / N) over [y-h, y+h) x [x-h, x+h) clipped to the image (N pixels).
+// A <= 4096 keeps N <= 2^24 and every window sum below 2^32, so the u32 table is exact for every window and there is no raster
+// path.  For N <= 65793 (N * 255 < 2^24) the floor is taken as cvt.rzi(div.rn((float)S, (float)N)) -- the defocus pass's
+// arithmetic, so f = 0, w = 0, A = K reproduces defocus bit for bit -- and above that as a u32 divide.
+// A kernel of its own rather than a fourth flag of effects_kernel: the box rule and the mean rule both differ, so the shared
+// kernel would branch on which caller it serves.
+// ---------------------------------------------------------------------------
+template <bool ALIGNED>
+__global__ void __launch_bounds__(256)
+refocus_kernel(const uint8_t *__restrict__ orig, size_t origPitch, const float *__restrict__ depth, size_t depthPitch,
+               uint8_t *__restrict__ out, size_t outPitch, const uint4 *__restrict__ sat, int rows, int cols,
+               float focus, const float *__restrict__ focusAt, float band, int aperture)
+{
+    const int x4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    const int y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (x4 >= cols || y >= rows) return;
+    const int n = min(4, cols - x4);
+    // "click to focus": the depth under the chosen pixel, read here so that no host round trip sits between solve and refocus
+    if (focusAt) focus = fminf(fmaxf(__ldg(focusAt), 0.0f), 255.0f);
+
+    unsigned int c[4][3];
+    load_bgr4<ALIGNED>(orig + (size_t)y * origPitch + 3 * x4, n, c);
+    float d[4];
+    {
+        const float *dRow = (const float *)((const char *)depth + (size_t)y * depthPitch) + x4;
+        if (ALIGNED && n == 4) {
+            const float4 v = __ldg((const float4 *)dRow);
+            d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
+        } else {
+#pragma unroll
+            for (int i = 0; i < 4; i++) d[i] = (i < n) ? __ldg(dRow + i) : 0.0f;
+        }
+    }
+
+    const int satPitch = cols + 1;
+    unsigned int o[4][3];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int x = x4 + i;
+        const float dc = fminf(fmaxf(d[i], 0.0f), 255.0f);
+        const float e = fmaxf(__fsub_rn(fabsf(__fsub_rn(dc, focus)), band), 0.0f);
+        const int a = __double2int_rz(__ddiv_rn((double)__fmul_rn((float)aperture, e), 255.0));
+        const int h = a / 2;
+        o[i][0] = c[i][0]; o[i][1] = c[i][1]; o[i][2] = c[i][2];
+        if (i < n && h > 0) {
+            const int x0 = max(x - h, 0), x1 = min(x + h, cols);
+            const int y0 = max(y - h, 0), y1 = min(y + h, rows);
+            const unsigned int count = (unsigned int)((x1 - x0) * (y1 - y0));
+            const uint4 s11 = sat_at(sat, nullptr, satPitch, y1, x1);
+            const uint4 s01 = sat_at(sat, nullptr, satPitch, y0, x1);
+            const uint4 s10 = sat_at(sat, nullptr, satPitch, y1, x0);
+            const uint4 s00 = sat_at(sat, nullptr, satPitch, y0, x0);
+            const unsigned int sb = s11.x - s01.x - s10.x + s00.x;
+            const unsigned int sg = s11.y - s01.y - s10.y + s00.y;
+            const unsigned int sr = s11.z - s01.z - s10.z + s00.z;
+            if (count <= 65793u) {
+                const float fc = (float)count;
+                o[i][0] = f2u8(__fdiv_rn((float)sb, fc));
+                o[i][1] = f2u8(__fdiv_rn((float)sg, fc));
+                o[i][2] = f2u8(__fdiv_rn((float)sr, fc));
+            } else {
+                o[i][0] = sb / count; o[i][1] = sg / count; o[i][2] = sr / count;
+            }
+        }
+    }
+    store_bgr4<ALIGNED>(out + (size_t)y * outPitch + 3 * x4, n, o);
+}
+
+cudaError_t launch_refocus(cudaStream_t s, const void *scratch, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                           uint8_t *out, size_t outPitch, int rows, int cols, float focus, const float *focusAt, float band, int aperture)
+{
+    const uint4 *sat = (const uint4 *)scratch;
+    const bool al = aligned4(orig, origPitch) && aligned16(depth, depthPitch) && aligned4(out, outPitch);
+    dim3 block(32, 8);
+    dim3 grid(rtdd_div_up(rtdd_div_up(cols, 4), block.x), rtdd_div_up(rows, block.y));
+    if (al)
+        refocus_kernel<true><<<grid, block, 0, s>>>(orig, origPitch, depth, depthPitch, out, outPitch, sat, rows, cols, focus, focusAt, band, aperture);
+    else
+        refocus_kernel<false><<<grid, block, 0, s>>>(orig, origPitch, depth, depthPitch, out, outPitch, sat, rows, cols, focus, focusAt, band, aperture);
+    return cudaGetLastError();
+}
+
 }  // namespace rtdd

@@ -1341,6 +1341,37 @@ int rtdd_defocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const flo
     return 0;
 }
 
+// Refocus parameters shared by rtdd_refocus and rtdd_frame_refocus: band half-width finite and >= 0; aperture <= 4096 after a
+// negative one has been replaced by the reference's K for the image size.  (The focus depth is checked by the callers: the frame
+// form may take it from the device instead.)
+static bool refocus_params_ok(float depthOfField, int *aperture, int rows, int cols)
+{
+    if (*aperture < 0) *aperture = rtdd::defocus_kernel_size(rows, cols);
+    return isfinite(depthOfField) && depthOfField >= 0.0f && *aperture <= RTDD_REFOCUS_MAX_APERTURE;
+}
+
+static bool focus_depth_ok(float f) { return f >= 0.0f && f <= 255.0f; }      // false for NaN
+
+int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                 uint8_t *out, size_t outPitch, int rows, int cols, float focusDepth, float depthOfField, int aperture)
+{
+    if (!ctx) return RTDD_E_ARG;
+    if (!orig || !depth || !out || rows < 0 || cols < 0 || origPitch < (size_t)cols * 3 || outPitch < (size_t)cols * 3 ||
+        depthPitch < (size_t)cols * sizeof(float) || !focus_depth_ok(focusDepth) || !refocus_params_ok(depthOfField, &aperture, rows, cols))
+        return rtdd_fail(ctx, RTDD_E_ARG, "rtdd_refocus");
+    if (rows == 0 || cols == 0) return 0;
+    DeviceGuard guard(ctx->device);
+    int rc = ensure_sat(ctx, rows, cols);
+    if (rc) return rc;
+    ctx->frameSatValid = false;            // the scratch is about to hold the table of the caller's image
+    RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, orig, origPitch, rows, cols), "rtdd_refocus (summed-area table)");
+    ctx->launches += 4;
+    RTDD_TRY(rtdd::launch_refocus(ctx->stream, ctx->satScratch, orig, origPitch, depth, depthPitch, out, outPitch, rows, cols,
+                                  focusDepth, nullptr, depthOfField, aperture), "rtdd_refocus");
+    ctx->launches++;
+    return 0;
+}
+
 int rtdd_effects_fused(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const uint8_t *gray, size_t grayPitch,
                        const float *depth, size_t depthPitch, uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch,
                        uint8_t *defocus, size_t defocusPitch, int rows, int cols)
@@ -1850,6 +1881,35 @@ int rtdd_frame_effects(rtdd_ctx *ctx, uint8_t *desat, size_t desatPitch, uint8_t
         RTDD_TRY(rtdd::launch_haze(s, ctx->bgr, ctx->bgrPitch, F.depth, F.depthPitch, haze, hazePitch, rows, cols), "rtdd_frame_effects (haze)");
         ctx->launches++;
     }
+    return 0;
+}
+
+// Refocus of the frame's own image by its solved level-0 depth, over the summed-area table rtdd_frame_effects caches too.  A focus
+// point makes the kernel read the depth under it, so a captured graph of this call follows every later solve.
+int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX, int focusY, float focusDepth,
+                       float depthOfField, int aperture)
+{
+    if (!ctx) return RTDD_E_ARG;
+    if (!ctx->imageSet) return rtdd_fail(ctx, RTDD_E_STATE, "rtdd_frame_refocus");
+    const int rows = ctx->rows, cols = ctx->cols;
+    const bool byDepth = focusX == -1 && focusY == -1;
+    const bool pointOk = focusX >= 0 && focusX < cols && focusY >= 0 && focusY < rows;
+    if (!out || outPitch < (size_t)cols * 3 || !(byDepth ? focus_depth_ok(focusDepth) : pointOk) ||
+        !refocus_params_ok(depthOfField, &aperture, rows, cols))
+        return rtdd_fail(ctx, RTDD_E_ARG, "rtdd_frame_refocus");
+    DeviceGuard guard(ctx->device);
+    RtddFrameLevel &F = ctx->fl[0];
+    const float *focusAt = byDepth ? nullptr : (const float *)((const char *)F.depth + (size_t)focusY * F.depthPitch) + focusX;
+    int rc = ensure_sat(ctx, rows, cols);
+    if (rc) return rc;
+    if (!ctx->frameSatValid) {
+        RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, rows, cols), "rtdd_frame_refocus (summed-area table)");
+        ctx->frameSatValid = true;
+        ctx->launches += 4;
+    }
+    RTDD_TRY(rtdd::launch_refocus(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, F.depth, F.depthPitch, out, outPitch, rows, cols,
+                                  byDepth ? focusDepth : 0.0f, focusAt, depthOfField, aperture), "rtdd_frame_refocus");
+    ctx->launches++;
     return 0;
 }
 

@@ -280,5 +280,10 @@ cudaError_t launch_defocus(cudaStream_t s, void *scratch, const uint8_t *orig, s
                            const float *depth, size_t depthPitch, uint8_t *defocus, size_t defocusPitch,
                            uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch,
                            int rows, int cols, int *launched, bool buildSat = true, int yBegin = 0, int yEnd = -1, int satRow0 = 0, int satRows = -1);
+// depth-of-field refocus over a summed-area table that launch_sat_build left in `scratch` (one launch).  focusAt != null: the focus
+// is the clamped depth at that device address, read by the kernel, and `focus` is ignored.  0 <= aperture <= RTDD_REFOCUS_MAX_APERTURE.
+#define RTDD_REFOCUS_MAX_APERTURE 4096     // largest box side: windows stay <= 2^24 pixels, window sums < 2^32
+cudaError_t launch_refocus(cudaStream_t s, const void *scratch, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                           uint8_t *out, size_t outPitch, int rows, int cols, float focus, const float *focusAt, float band, int aperture);
 
 }  // namespace rtdd

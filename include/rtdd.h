@@ -279,6 +279,33 @@ int rtdd_effects_rows(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, cons
 int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
                  uint8_t *out, size_t outPitch, int rows, int cols, float focusDepth, float depthOfField, int aperture);
 
+/* Extension, no reference counterpart: stereo views of a device image by a device depth plane, the image taken as the centre view
+ * (see DESIGN.md §7).  Depth 0 is near, 255 far.  convergenceDepth c in [0, 255] is the zero-parallax plane; maxDisparity D, in
+ * [0, RTDD_STEREO_MAX_DISPARITY] pixels, is the parallax of a depth 255 away from it.  Per source pixel (x, y):
+ *   d' = fminf(fmaxf(d, 0), 255) (NaN -> 0; -0 counts as +0);
+ *   s = cvt.rzi.s32.f64((double)__fmul_rn((float)D, __fsub_rn(d', c)) / 255.0), the signed parallax in [-D, D];
+ *   hL = s / 2 (C division, toward zero), hR = s - hL; the pixel lands on tL = x - hL in the left view and on tR = x + hR in the
+ *   right one (tR - tL = s: farther than c is behind the screen, nearer is in front).  Targets outside [0, cols) are dropped.
+ * Per view, row and target column t:
+ *   covered (a source lands on t): the source with the smallest d' wins (the nearest occludes) and t shows orig[y][winner].
+ *     Two sources with equal d' have equal s, so they never land on the same target: the winner is unique, every order of
+ *     evaluation gives the same bytes, and an atomic minimum over d' is exact;
+ *   a hole, with l and r the nearest covered targets left and right of t in the row: t shows the view's pixel at l when l exists
+ *     and (r does not, or d' of l's winner >= d' of r's winner), otherwise the view's pixel at r -- the farther side, the
+ *     background, fills the hole, ties to the left;
+ *   a row with no covered target (D large against cols): orig[y][t].
+ * The anaglyph (red-cyan) takes B and G from the right view and R from the left one.  D = 0, or every depth equal to c, gives
+ * left = right = anaglyph = orig; a constant depth d0 != c shifts the image by -hL / +hR and repeats the nearest covered column.
+ * Outputs are device BGR planes with byte pitches >= 3 x cols; any of them may be NULL, not all three.  Side by side is pointers
+ * alone: left = buf, right = buf + 3 x cols, both with pitch 6 x cols.  Outputs must not overlap orig or depth.  depth is an fp32
+ * plane: its address and pitch are multiples of 4.  cols <= RTDD_STEREO_MAX_COLS (one row is held on chip).  One launch, no
+ * context scratch. */
+#define RTDD_STEREO_MAX_DISPARITY 1024
+#define RTDD_STEREO_MAX_COLS      16384
+int rtdd_stereo(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch, uint8_t *anaglyph, size_t anaglyphPitch,
+                int rows, int cols, float convergenceDepth, int maxDisparity);
+
 /* ---- pyramid ops either side of the path (SURVEY.md section 8f) ------------------- */
 
 /* cv::cvtColor(BGR2GRAY)                 ref: src/main.cpp:111,138 */
@@ -347,6 +374,13 @@ int rtdd_frame_effects(rtdd_ctx *ctx, uint8_t *desat, size_t desatPitch, uint8_t
  * captured from this call follows every later solve;  focusX = focusY = -1: focus = focusDepth. */
 int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX, int focusY, float focusDepth,
                        float depthOfField, int aperture);
+/* rtdd_stereo on the frame context's own image and solved level-0 depth (1 launch; the summed-area table cached for
+ * rtdd_frame_effects / rtdd_frame_refocus is left valid).
+ * convergenceX, convergenceY inside the image: c = clamped depth under that pixel, read on the device (convergenceDepth ignored)
+ * -- a graph captured from this call follows every later solve;  convergenceX = convergenceY = -1: c = convergenceDepth. */
+int rtdd_frame_stereo(rtdd_ctx *ctx, uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch,
+                      uint8_t *anaglyph, size_t anaglyphPitch, int convergenceX, int convergenceY,
+                      float convergenceDepth, int maxDisparity);
 /* ref: src/main.cpp:46-62 -- brush stroke into the context's level-0 annotation planes */
 int rtdd_frame_paint(rtdd_ctx *ctx, int x, int y, int scribbleColor, int scribbleRadius);
 /* device pointers/pitches of the context-owned planes (for effects, tests, downloads) */

@@ -72,6 +72,8 @@ SIGNATURES = {
     "rtdd_effects_fused": (i32, [vp, vp, sz, vp, sz, vp, sz, vp, sz, vp, sz, vp, sz, i32, i32]),
     "rtdd_refocus": (i32, [vp, vp, sz, vp, sz, vp, sz, i32, i32, f32, f32, i32]),
     "rtdd_frame_refocus": (i32, [vp, vp, sz, i32, i32, f32, f32, i32]),
+    "rtdd_stereo": (i32, [vp, vp, sz, vp, sz, vp, sz, vp, sz, vp, sz, i32, i32, f32, i32]),
+    "rtdd_frame_stereo": (i32, [vp, vp, sz, vp, sz, vp, sz, i32, i32, f32, i32]),
     "rtdd_bgr2gray": (i32, [vp, vp, sz, vp, sz, i32, i32]),
     "rtdd_pyrdown_gray": (i32, [vp, vp, sz, i32, i32, vp, sz]),
     "rtdd_pyrup_depth": (i32, [vp, vp, sz, i32, i32, vp, sz, i32, i32]),

@@ -219,6 +219,16 @@ class DepthDiffusion:
         self._ck(lib.rtdd_refocus(self._h, _ptr(orig), _pitch(orig), _ptr(depth), _pitch(depth), _ptr(out), _pitch(out), rows, cols,
                                   float(focus_depth), float(depth_of_field), -1 if aperture is None else int(aperture)))
 
+    def stereo(self, orig, depth, left=None, right=None, anaglyph=None, convergence_depth=0.0, max_disparity=32):
+        """Extension (no reference counterpart): left and right views of `orig` by `depth` (0 near, 255 far) and their red-cyan
+        anaglyph, into device BGR planes, any of them None but not all.  Depth `convergence_depth` sits on the screen; depths 255
+        away from it get `max_disparity` pixels of parallax.  Side by side: left = buf[:, :3*cols], right = buf[:, 3*cols:] of one
+        rows x 6*cols plane.  See rtdd_stereo in include/rtdd.h."""
+        rows, cols = depth.shape
+        self._ck(lib.rtdd_stereo(self._h, _ptr(orig), _pitch(orig), _ptr(depth), _pitch(depth), _ptr(left), _pitch(left),
+                                 _ptr(right), _pitch(right), _ptr(anaglyph), _pitch(anaglyph), rows, cols,
+                                 float(convergence_depth), int(max_disparity)))
+
     # -- pyramid ops ---------------------------------------------------------------
     def bgr2gray(self, bgr, gray):
         rows, cols = gray.shape
@@ -316,6 +326,18 @@ class DepthDiffusion:
             fx, fy, fd = int(focus_point[0]), int(focus_point[1]), float("nan")
         self._ck(lib.rtdd_frame_refocus(self._h, _ptr(out), _pitch(out), fx, fy, fd, float(depth_of_field),
                                         -1 if aperture is None else int(aperture)))
+
+    def frame_stereo(self, left=None, right=None, anaglyph=None, convergence_point=None, convergence_depth=None, max_disparity=32):
+        """stereo() of the frame's own image by its solved depth.  Give exactly one of convergence_point = (x, y), whose depth is
+        read on the GPU (no host round trip, so a captured graph follows later solves), and convergence_depth."""
+        if (convergence_point is None) == (convergence_depth is None):
+            raise ValueError("frame_stereo: give exactly one of convergence_point and convergence_depth")
+        if convergence_point is None:
+            cx, cy, cd = -1, -1, float(convergence_depth)
+        else:                 # NaN: a point of (-1, -1) is refused like any other point outside the image
+            cx, cy, cd = int(convergence_point[0]), int(convergence_point[1]), float("nan")
+        self._ck(lib.rtdd_frame_stereo(self._h, _ptr(left), _pitch(left), _ptr(right), _pitch(right), _ptr(anaglyph), _pitch(anaglyph),
+                                       cx, cy, cd, int(max_disparity)))
 
     PLANE_DEPTH, PLANE_GRAY, PLANE_SCRIBBLE, PLANE_EDITED, PLANE_BGR, PLANE_DEPTH_U8 = range(6)
 

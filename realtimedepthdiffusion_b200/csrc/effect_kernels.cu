@@ -682,4 +682,185 @@ cudaError_t launch_refocus(cudaStream_t s, const void *scratch, const uint8_t *o
     return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------
+// stereo (extension, no reference counterpart): left and right views and a red-cyan anaglyph, the image taken as the centre view.
+//   d' = clamp(d, 0, 255) (NaN -> 0, -0 -> +0); s = cvt.rzi.s32.f64((double)((float)D * (d' - c)) / 255.0); hL = s / 2; hR = s - hL.
+//   Source x lands on tL = x - hL in the left view and on tR = x + hR in the right one.  A target column takes the landing source
+//   with the smallest d'; a hole takes the covered neighbour (nearest on each side) whose winner is farther, the left one on a tie;
+//   a row with no covered column keeps the image's own pixels.
+// Every output row depends on its own source row only, so one CTA takes one row and keeps the row's per-column state in shared
+// memory, per view: a z-buffer of d' bits (d' >= 0 with -0 made +0, so the bits order like the values), the winning source
+// column, and a two-level bitmap of covered columns (a bit per column, a bit per non-empty word) that finds the nearest covered
+// column on either side of a hole in a few instructions, with no scan over the row.  Sources of equal d' have equal s and so
+// never land on the same target: the winner of a column is unique, and a u32 atomicMin of the bits followed by "the source whose
+// bits equal the minimum writes its x" is exact in any order.  12 B per column + the bitmaps: 196 KB at 16384 columns.
+// ---------------------------------------------------------------------------
+constexpr int STEREO_THREADS = 512;
+constexpr unsigned int STEREO_EMPTY = 0xFFFFFFFFu;       // z-buffer value of a column no source landed on
+
+__device__ __forceinline__ float stereo_depth(float d) { return __fadd_rn(fminf(fmaxf(d, 0.0f), 255.0f), 0.0f); }
+
+// s = cvt.rzi.s32.f64((double)q / 255.0) with q = __fmul_rn(D, d' - c), taken as trunc(q) / 255 in integers: the same value for
+// every float q, because the quotient is an integer n exactly when q = 255 n, and otherwise lies at least 2^-31 from every integer
+// (|q| >= 1 is a multiple of 2^-23) while its fp64 rounding error is below 2^-42 (|q| / 255 <= 1024).  No fp64 divide in the
+// loop, and no call into its slow path.
+__device__ __forceinline__ int stereo_parallax(float dc, float conv, float D)
+{
+    return __float2int_rz(__fmul_rn(D, __fsub_rn(dc, conv))) / 255;
+}
+
+// largest covered column <= t, or -1.  b0: a bit per column; b1: a bit per non-zero word of b0; top: a bit per non-zero word of b1
+__device__ __forceinline__ int stereo_prev(const unsigned int *b0, const unsigned int *b1, unsigned int top, int t)
+{
+    int w = t >> 5;
+    unsigned int m = b0[w] & (0xFFFFFFFFu >> (31 - (t & 31)));
+    if (m) return (w << 5) + 31 - __clz(m);
+    int w1 = w >> 5;
+    m = b1[w1] & ((1u << (w & 31)) - 1u);
+    if (!m) {
+        const unsigned int mt = top & ((1u << w1) - 1u);
+        if (!mt) return -1;
+        w1 = 31 - __clz(mt);
+        m = b1[w1];
+    }
+    w = (w1 << 5) + 31 - __clz(m);
+    return (w << 5) + 31 - __clz(b0[w]);
+}
+
+// smallest covered column >= t, or -1
+__device__ __forceinline__ int stereo_next(const unsigned int *b0, const unsigned int *b1, unsigned int top, int t)
+{
+    int w = t >> 5;
+    unsigned int m = b0[w] & (0xFFFFFFFFu << (t & 31));
+    if (m) return (w << 5) + __ffs(m) - 1;
+    int w1 = w >> 5;
+    m = b1[w1] & (0xFFFFFFFEu << (w & 31));
+    if (!m) {
+        const unsigned int mt = top & (0xFFFFFFFEu << w1);
+        if (!mt) return -1;
+        w1 = __ffs(mt) - 1;
+        m = b1[w1];
+    }
+    w = (w1 << 5) + __ffs(m) - 1;
+    return (w << 5) + __ffs(b0[w]) - 1;
+}
+
+// the source column whose pixel one view shows at target column t
+__device__ __forceinline__ int stereo_source(const unsigned int *key, const unsigned short *win, const unsigned int *b0,
+                                             const unsigned int *b1, unsigned int top, int t)
+{
+    if (key[t] != STEREO_EMPTY) return win[t];
+    const int l = stereo_prev(b0, b1, top, t), r = stereo_next(b0, b1, top, t);
+    if (r < 0) return l < 0 ? t : win[l];
+    return (l >= 0 && key[l] >= key[r]) ? win[l] : win[r];
+}
+
+static size_t stereo_smem_bytes(int cols)
+{
+    return (size_t)12 * cols + (size_t)8 * ((cols + 31) / 32) + 128;
+}
+
+template <bool ALIGNED>
+__global__ void __launch_bounds__(STEREO_THREADS)
+stereo_kernel(const uint8_t *__restrict__ orig, size_t origPitch, const float *__restrict__ depth, size_t depthPitch,
+              uint8_t *__restrict__ left, size_t leftPitch, uint8_t *__restrict__ right, size_t rightPitch,
+              uint8_t *__restrict__ anaglyph, size_t anaglyphPitch, int cols, float conv, const float *__restrict__ convAt, int maxDisparity)
+{
+    extern __shared__ __align__(16) unsigned char stereo_smem[];
+    const int W = (cols + 31) >> 5, W1 = (W + 31) >> 5;            // W1 <= 16 for cols <= 16384
+    unsigned int *key = (unsigned int *)stereo_smem;                // [2][cols] view 0 = left, 1 = right
+    unsigned int *b0 = key + 2 * cols;                              // [2][W]
+    unsigned int *b1 = b0 + 2 * W;                                  // [2][16]
+    unsigned short *win = (unsigned short *)(b1 + 32);              // [2][cols]
+    const int y = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const bool needL = left || anaglyph, needR = right || anaglyph;
+    // "click to converge": the depth under the chosen pixel, read here so that no host round trip sits between solve and stereo
+    if (convAt) conv = stereo_depth(__ldg(convAt));
+    const float D = (float)maxDisparity;
+    const uint8_t *src = orig + (size_t)y * origPitch;
+    const float *dRow = (const float *)((const char *)depth + (size_t)y * depthPitch);
+
+    for (int t = tid; t < 2 * cols; t += STEREO_THREADS) key[t] = STEREO_EMPTY;
+    __syncthreads();
+    for (int x = tid; x < cols; x += STEREO_THREADS) {
+        const float dc = stereo_depth(__ldg(dRow + x));
+        const int s = stereo_parallax(dc, conv, D), hL = s / 2;
+        const int tL = x - hL, tR = x + (s - hL);
+        if (needL && (unsigned)tL < (unsigned)cols) atomicMin(key + tL, __float_as_uint(dc));
+        if (needR && (unsigned)tR < (unsigned)cols) atomicMin(key + cols + tR, __float_as_uint(dc));
+    }
+    __syncthreads();
+    for (int x = tid; x < cols; x += STEREO_THREADS) {             // the row's depth is in L1 now
+        const float dc = stereo_depth(__ldg(dRow + x));
+        const int s = stereo_parallax(dc, conv, D), hL = s / 2;
+        const int tL = x - hL, tR = x + (s - hL);
+        if (needL && (unsigned)tL < (unsigned)cols && key[tL] == __float_as_uint(dc)) win[tL] = (unsigned short)x;
+        if (needR && (unsigned)tR < (unsigned)cols && key[cols + tR] == __float_as_uint(dc)) win[cols + tR] = (unsigned short)x;
+    }
+    for (int t = tid; t < 32 * W; t += STEREO_THREADS) {            // whole warps: both bounds are multiples of 32
+        const unsigned int mL = __ballot_sync(0xFFFFFFFFu, t < cols && key[t] != STEREO_EMPTY);
+        const unsigned int mR = __ballot_sync(0xFFFFFFFFu, t < cols && key[cols + t] != STEREO_EMPTY);
+        if (lane == 0) { b0[t >> 5] = mL; b0[W + (t >> 5)] = mR; }
+    }
+    __syncthreads();
+    for (int w = tid; w < 32 * W1; w += STEREO_THREADS) {
+        const unsigned int mL = __ballot_sync(0xFFFFFFFFu, w < W && b0[w] != 0u);
+        const unsigned int mR = __ballot_sync(0xFFFFFFFFu, w < W && b0[W + w] != 0u);
+        if (lane == 0) { b1[w >> 5] = mL; b1[16 + (w >> 5)] = mR; }
+    }
+    __syncthreads();
+    const unsigned int topL = __ballot_sync(0xFFFFFFFFu, lane < W1 && b1[lane] != 0u);
+    const unsigned int topR = __ballot_sync(0xFFFFFFFFu, lane < W1 && b1[16 + lane] != 0u);
+
+    for (int x4 = 4 * tid; x4 < cols; x4 += 4 * STEREO_THREADS) {
+        const int n = min(4, cols - x4);
+        unsigned int cl[4][3], cr[4][3];
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            cl[i][0] = cl[i][1] = cl[i][2] = cr[i][0] = cr[i][1] = cr[i][2] = 0u;
+            if (i < n) {
+                if (needL) {
+                    const uint8_t *p = src + 3 * stereo_source(key, win, b0, b1, topL, x4 + i);
+                    cl[i][0] = __ldg(p); cl[i][1] = __ldg(p + 1); cl[i][2] = __ldg(p + 2);
+                }
+                if (needR) {
+                    const uint8_t *p = src + 3 * stereo_source(key + cols, win + cols, b0 + W, b1 + 16, topR, x4 + i);
+                    cr[i][0] = __ldg(p); cr[i][1] = __ldg(p + 1); cr[i][2] = __ldg(p + 2);
+                }
+            }
+        }
+        if (left) store_bgr4<ALIGNED>(left + (size_t)y * leftPitch + 3 * x4, n, cl);
+        if (right) store_bgr4<ALIGNED>(right + (size_t)y * rightPitch + 3 * x4, n, cr);
+        if (anaglyph) {
+#pragma unroll
+            for (int i = 0; i < 4; i++) cr[i][2] = cl[i][2];            // B, G of the right view, R of the left one
+            store_bgr4<ALIGNED>(anaglyph + (size_t)y * anaglyphPitch + 3 * x4, n, cr);
+        }
+    }
+}
+
+cudaError_t configure_stereo()
+{
+    const int bytes = (int)stereo_smem_bytes(RTDD_STEREO_MAX_COLS);
+    cudaError_t e = cudaFuncSetAttribute(stereo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(stereo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    return e;
+}
+
+cudaError_t launch_stereo(cudaStream_t s, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                          uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch, uint8_t *anaglyph, size_t anaglyphPitch,
+                          int rows, int cols, float conv, const float *convAt, int maxDisparity)
+{
+    const bool al = (!left || aligned4(left, leftPitch)) && (!right || aligned4(right, rightPitch)) &&
+                    (!anaglyph || aligned4(anaglyph, anaglyphPitch));
+    const size_t smem = stereo_smem_bytes(cols);
+    if (al)
+        stereo_kernel<true><<<rows, STEREO_THREADS, smem, s>>>(orig, origPitch, depth, depthPitch, left, leftPitch, right, rightPitch,
+                                                               anaglyph, anaglyphPitch, cols, conv, convAt, maxDisparity);
+    else
+        stereo_kernel<false><<<rows, STEREO_THREADS, smem, s>>>(orig, origPitch, depth, depthPitch, left, leftPitch, right, rightPitch,
+                                                                anaglyph, anaglyphPitch, cols, conv, convAt, maxDisparity);
+    return cudaGetLastError();
+}
+
 }  // namespace rtdd

@@ -575,6 +575,7 @@ static int create_impl(int rows, int cols, int levels, int device, const int *pl
     }
     build_tensor_maps(ctx);
     e = rtdd::configure_kernels();
+    if (e == cudaSuccess) e = rtdd::configure_stereo();
     for (int l = 0; l < levels && e == cudaSuccess; l++) {
         e = cudaEventCreate(&ctx->lv[l].evBegin);
         if (e == cudaSuccess) e = cudaEventCreate(&ctx->lv[l].evEnd);
@@ -1372,6 +1373,34 @@ int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const flo
     return 0;
 }
 
+// Stereo outputs shared by rtdd_stereo and rtdd_frame_stereo: at least one plane, each with a full row of BGR bytes; the maximum
+// disparity in [0, RTDD_STEREO_MAX_DISPARITY]; a row the kernel can hold.  (The convergence depth is checked by the callers.)
+static bool stereo_params_ok(const uint8_t *left, size_t leftPitch, const uint8_t *right, size_t rightPitch,
+                             const uint8_t *anaglyph, size_t anaglyphPitch, int cols, int maxDisparity)
+{
+    const size_t rowBytes = (size_t)cols * 3;
+    return (left || right || anaglyph) && (!left || leftPitch >= rowBytes) && (!right || rightPitch >= rowBytes) &&
+           (!anaglyph || anaglyphPitch >= rowBytes) && cols <= RTDD_STEREO_MAX_COLS &&
+           maxDisparity >= 0 && maxDisparity <= RTDD_STEREO_MAX_DISPARITY;
+}
+
+int rtdd_stereo(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch, uint8_t *anaglyph, size_t anaglyphPitch,
+                int rows, int cols, float convergenceDepth, int maxDisparity)
+{
+    if (!ctx) return RTDD_E_ARG;
+    if (!orig || !depth || rows < 0 || cols < 0 || origPitch < (size_t)cols * 3 || depthPitch < (size_t)cols * sizeof(float) ||
+        (((uintptr_t)depth | depthPitch) & 3u) || !focus_depth_ok(convergenceDepth) ||
+        !stereo_params_ok(left, leftPitch, right, rightPitch, anaglyph, anaglyphPitch, cols, maxDisparity))
+        return rtdd_fail(ctx, RTDD_E_ARG, "rtdd_stereo");
+    if (rows == 0 || cols == 0) return 0;
+    DeviceGuard guard(ctx->device);
+    RTDD_TRY(rtdd::launch_stereo(ctx->stream, orig, origPitch, depth, depthPitch, left, leftPitch, right, rightPitch, anaglyph, anaglyphPitch,
+                                 rows, cols, convergenceDepth, nullptr, maxDisparity), "rtdd_stereo");
+    ctx->launches++;
+    return 0;
+}
+
 int rtdd_effects_fused(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const uint8_t *gray, size_t grayPitch,
                        const float *depth, size_t depthPitch, uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch,
                        uint8_t *defocus, size_t defocusPitch, int rows, int cols)
@@ -1909,6 +1938,31 @@ int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX,
     }
     RTDD_TRY(rtdd::launch_refocus(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, F.depth, F.depthPitch, out, outPitch, rows, cols,
                                   byDepth ? focusDepth : 0.0f, focusAt, depthOfField, aperture), "rtdd_frame_refocus");
+    ctx->launches++;
+    return 0;
+}
+
+// Stereo views of the frame's own image by its solved level-0 depth.  Needs no scratch, so the summed-area table that
+// rtdd_frame_effects and rtdd_frame_refocus cache stays valid.  A convergence point makes the kernel read the depth under it, so a
+// captured graph of this call follows every later solve.
+int rtdd_frame_stereo(rtdd_ctx *ctx, uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch,
+                      uint8_t *anaglyph, size_t anaglyphPitch, int convergenceX, int convergenceY,
+                      float convergenceDepth, int maxDisparity)
+{
+    if (!ctx) return RTDD_E_ARG;
+    if (!ctx->imageSet) return rtdd_fail(ctx, RTDD_E_STATE, "rtdd_frame_stereo");
+    const int rows = ctx->rows, cols = ctx->cols;
+    const bool byDepth = convergenceX == -1 && convergenceY == -1;
+    const bool pointOk = convergenceX >= 0 && convergenceX < cols && convergenceY >= 0 && convergenceY < rows;
+    if (!(byDepth ? focus_depth_ok(convergenceDepth) : pointOk) ||
+        !stereo_params_ok(left, leftPitch, right, rightPitch, anaglyph, anaglyphPitch, cols, maxDisparity))
+        return rtdd_fail(ctx, RTDD_E_ARG, "rtdd_frame_stereo");
+    DeviceGuard guard(ctx->device);
+    RtddFrameLevel &F = ctx->fl[0];
+    const float *convAt = byDepth ? nullptr : (const float *)((const char *)F.depth + (size_t)convergenceY * F.depthPitch) + convergenceX;
+    RTDD_TRY(rtdd::launch_stereo(ctx->stream, ctx->bgr, ctx->bgrPitch, F.depth, F.depthPitch, left, leftPitch, right, rightPitch,
+                                 anaglyph, anaglyphPitch, rows, cols, byDepth ? convergenceDepth : 0.0f, convAt, maxDisparity),
+             "rtdd_frame_stereo");
     ctx->launches++;
     return 0;
 }

@@ -285,5 +285,13 @@ cudaError_t launch_defocus(cudaStream_t s, void *scratch, const uint8_t *orig, s
 #define RTDD_REFOCUS_MAX_APERTURE 4096     // largest box side: windows stay <= 2^24 pixels, window sums < 2^32
 cudaError_t launch_refocus(cudaStream_t s, const void *scratch, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
                            uint8_t *out, size_t outPitch, int rows, int cols, float focus, const float *focusAt, float band, int aperture);
+// stereo views and anaglyph (one launch, no scratch); any one or two of left / right / anaglyph may be null.  convAt != null: the
+// convergence depth is the clamped depth at that device address, read by the kernel, and `conv` is ignored.
+// 1 <= cols <= RTDD_STEREO_MAX_COLS, 0 <= maxDisparity <= RTDD_STEREO_MAX_DISPARITY.
+cudaError_t launch_stereo(cudaStream_t s, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
+                          uint8_t *left, size_t leftPitch, uint8_t *right, size_t rightPitch, uint8_t *anaglyph, size_t anaglyphPitch,
+                          int rows, int cols, float conv, const float *convAt, int maxDisparity);
+// the stereo kernel's shared-memory limit (a row of RTDD_STEREO_MAX_COLS columns); called next to configure_kernels
+cudaError_t configure_stereo();
 
 }  // namespace rtdd

@@ -275,7 +275,7 @@ int rtdd_effects_rows(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, cons
  * the exact mean of orig over [y-h, y+h) x [x-h, x+h) clipped to the image.  focusDepth in [0, 255]; depthOfField (the half-width
  * of the sharp band, depth units) finite and >= 0; aperture (the largest box side, pixels) <= 4096, a negative one selects the
  * reference defocus's K = (int)(0.025 x diagonal).  focusDepth = 0, depthOfField = 0, aperture = K gives rtdd_defocus's bytes
- * for every depth <= 255 while K <= 257.  Builds the summed-area table of orig (4 launches) and refocuses (1). */
+ * for every depth <= 255 while K <= 257.  Builds the summed-area table of orig (4 launches, 5 for cols > 16384) and refocuses (1). */
 int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const float *depth, size_t depthPitch,
                  uint8_t *out, size_t outPitch, int rows, int cols, float focusDepth, float depthOfField, int aperture);
 
@@ -369,7 +369,7 @@ int rtdd_frame_solve_band(rtdd_ctx *ctx, int maxIterations, int rowBegin, int ro
  * on the image only and is built once per rtdd_frame_set_image, not once per call. */
 int rtdd_frame_effects(rtdd_ctx *ctx, uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch, uint8_t *defocus, size_t defocusPitch);
 /* rtdd_refocus on the frame context's own image and solved level-0 depth, with the cached summed-area table (shared with
- * rtdd_frame_effects; built only when absent: 1 launch, else 5).
+ * rtdd_frame_effects): 1 launch, plus the table's 4 (5 for cols > 16384) when it is absent.
  * focusX, focusY inside the image: focus = clamped depth under that pixel, read on the device (focusDepth ignored) -- a graph
  * captured from this call follows every later solve;  focusX = focusY = -1: focus = focusDepth. */
 int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX, int focusY, float focusDepth,

@@ -550,7 +550,7 @@ size_t defocus_scratch_bytes(int rows, int cols)
 // (rtdd_frame_effects).  Tried: a single table pass (column sums kept in registers while one CTA per 8-row group walks
 // down and scans along x; table written once, no per-lookup offset) -- correct, but its serial rows with two CTA barriers
 // each made it slower than these three streaming passes (4K defocus 0.270 vs 0.248 ms), so it was not kept.
-cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig, size_t origPitch, int rows, int cols)
+cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig, size_t origPitch, int rows, int cols, int *launched)
 {
     uint4 *sat = (uint4 *)scratch;
     uint4 *aux = sat + (size_t)(rows + 1) * (cols + 1);
@@ -558,6 +558,7 @@ cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig,
     sat_group_colsums_kernel<<<dim3(rtdd_div_up(rtdd_div_up(cols, 4), 128), groups), 128, 0, s>>>(orig, origPitch, aux, rows, cols);
     sat_group_prefix_kernel<<<groups, 256, 0, s>>>(aux, cols);
     sat_aux_kernel<<<rtdd_div_up(cols + 1, 32), 256, 0, s>>>(aux, groups, cols);
+    *launched = 4;
     if (cols <= 4096) {
         sat_fused_kernel<1><<<groups, 1024, 0, s>>>(orig, origPitch, sat, aux, rows, cols);
     } else if (cols <= 8192) {
@@ -567,6 +568,7 @@ cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig,
     } else {                 // wider than 16384 columns: the two streaming passes of round 1
         sat_rows_kernel<<<rows, 256, 0, s>>>(orig, origPitch, sat, rows, cols);
         sat_cols_kernel<<<dim3(rtdd_div_up(cols + 1, 128), groups), 128, 0, s>>>(sat, aux, rows, cols);
+        *launched = 5;
     }
     return cudaGetLastError();
 }
@@ -584,9 +586,8 @@ cudaError_t launch_defocus(cudaStream_t s, void *scratch, const uint8_t *orig, s
     const int K = defocus_kernel_size(rows, cols);
     *launched = 0;
     if (buildSat) {
-        cudaError_t e = launch_sat_build(s, scratch, orig + (size_t)satRow0 * origPitch, origPitch, satRows, cols);
+        cudaError_t e = launch_sat_build(s, scratch, orig + (size_t)satRow0 * origPitch, origPitch, satRows, cols, launched);
         if (e != cudaSuccess) return e;
-        *launched = 4;
     }
     *launched += 1;
     if (desat && haze)

@@ -1365,8 +1365,9 @@ int rtdd_refocus(rtdd_ctx *ctx, const uint8_t *orig, size_t origPitch, const flo
     int rc = ensure_sat(ctx, rows, cols);
     if (rc) return rc;
     ctx->frameSatValid = false;            // the scratch is about to hold the table of the caller's image
-    RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, orig, origPitch, rows, cols), "rtdd_refocus (summed-area table)");
-    ctx->launches += 4;
+    int launched = 0;
+    RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, orig, origPitch, rows, cols, &launched), "rtdd_refocus (summed-area table)");
+    ctx->launches += launched;
     RTDD_TRY(rtdd::launch_refocus(ctx->stream, ctx->satScratch, orig, origPitch, depth, depthPitch, out, outPitch, rows, cols,
                                   focusDepth, nullptr, depthOfField, aperture), "rtdd_refocus");
     ctx->launches++;
@@ -1932,9 +1933,10 @@ int rtdd_frame_refocus(rtdd_ctx *ctx, uint8_t *out, size_t outPitch, int focusX,
     int rc = ensure_sat(ctx, rows, cols);
     if (rc) return rc;
     if (!ctx->frameSatValid) {
-        RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, rows, cols), "rtdd_frame_refocus (summed-area table)");
+        int launched = 0;
+        RTDD_TRY(rtdd::launch_sat_build(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, rows, cols, &launched), "rtdd_frame_refocus (summed-area table)");
         ctx->frameSatValid = true;
-        ctx->launches += 4;
+        ctx->launches += launched;
     }
     RTDD_TRY(rtdd::launch_refocus(ctx->stream, ctx->satScratch, ctx->bgr, ctx->bgrPitch, F.depth, F.depthPitch, out, outPitch, rows, cols,
                                   byDepth ? focusDepth : 0.0f, focusAt, depthOfField, aperture), "rtdd_frame_refocus");

@@ -274,8 +274,9 @@ cudaError_t launch_haze(cudaStream_t s, const uint8_t *orig, size_t origPitch, c
                         uint8_t *out, size_t outPitch, int rows, int cols);
 int defocus_kernel_size(int rows, int cols);
 size_t defocus_scratch_bytes(int rows, int cols);
+// summed-area table of orig into `scratch`; *launched = number of kernels launched (4, or 5 wider than 16384 columns)
+cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig, size_t origPitch, int rows, int cols, int *launched);
 // desat/haze may be null (defocus only); returns number of kernels launched through *launched
-cudaError_t launch_sat_build(cudaStream_t s, void *scratch, const uint8_t *orig, size_t origPitch, int rows, int cols);
 cudaError_t launch_defocus(cudaStream_t s, void *scratch, const uint8_t *orig, size_t origPitch, const uint8_t *gray, size_t grayPitch,
                            const float *depth, size_t depthPitch, uint8_t *defocus, size_t defocusPitch,
                            uint8_t *desat, size_t desatPitch, uint8_t *haze, size_t hazePitch,

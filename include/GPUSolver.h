@@ -14,7 +14,8 @@
 void GPUAllocateDeviceMemory(int rows, int cols, int levels);
 // ref GPUSolver.h:7 / GPUSolver.cu:56-71
 void GPUFreeDeviceMemory(int levels);
-// ref GPUSolver.h:8 / GPUSolver.cu:264-272 -- w[d] = expf(-beta*d), d = 0..255
+// ref GPUSolver.h:8 / GPUSolver.cu:264-272 -- w[d] = expf(-beta*d), d = 0..255.  Deviation: a negative, NaN or
+// infinite beta is refused (error printed, previous table kept), see rtdd_load_weights.
 void GPULoadWeights(float beta);
 // ref GPUSolver.h:9-10 / GPUSolver.cu:274-316 -- one pyramid level, depthImage updated in
 // place; all pointers are device pointers with byte pitches; beta and tolerance are accepted

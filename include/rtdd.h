@@ -49,7 +49,10 @@ int rtdd_create(int rows, int cols, int levels, int device, rtdd_ctx **out);
 int rtdd_create_strip(int rows, int cols, int levels, int device, int nranks, int halo, long long minStripPixels, rtdd_ctx **out);
 /* replaces GPUFreeDeviceMemory(levels)                    ref: include/GPUSolver.h:7, src/GPUSolver.cu:56-71 */
 int rtdd_destroy(rtdd_ctx *ctx);
-/* replaces GPULoadWeights(beta)                           ref: include/GPUSolver.h:8, src/GPUSolver.cu:264-272 */
+/* replaces GPULoadWeights(beta)                           ref: include/GPUSolver.h:8, src/GPUSolver.cu:264-272
+ * w[i] = expf(-beta * i) for i = 0..255 (host fp32), w[256] = 0.  Deviation: beta < 0 (weights above 1) and NaN or
+ * infinite beta (NaN weights) return RTDD_E_ARG and leave the previously loaded table, or none, in force; -0.0 is accepted.
+ * The table may be reloaded at any time: later solves, cached graphs included, use the new one. */
 int rtdd_load_weights(rtdd_ctx *ctx, float beta);
 /* stream = a cudaStream_t (NULL restores the context's own stream). */
 int rtdd_set_stream(rtdd_ctx *ctx, void *stream);

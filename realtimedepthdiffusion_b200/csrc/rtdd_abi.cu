@@ -7,6 +7,7 @@
 #include "rtdd_internal.h"
 
 #include <math.h>
+#include <cmath>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -611,6 +612,10 @@ int rtdd_destroy(rtdd_ctx *ctx)
 int rtdd_load_weights(rtdd_ctx *ctx, float beta)
 {
     if (!ctx) return RTDD_E_ARG;
+    // Deviation: the reference accepts any beta.  A negative one gives weights above 1 (sums above 8, outside the range the
+    // sweeps' branch-free division is proven for, which the cluster kernel does not check), a non-finite one NaN weights;
+    // neither has an edge-stopping meaning.  Refused before the table is touched, so the previous one stays in force.
+    if (!(beta >= 0.0f) || !std::isfinite(beta)) return rtdd_fail(ctx, RTDD_E_ARG, "rtdd_load_weights (beta must be finite and >= 0)");
     DeviceGuard guard(ctx->device);
     // ref: src/GPUSolver.cu:266-268 -- host expf, fp32
     for (int w = 0; w < 256; w++) ctx->hLut[w] = expf(-beta * w);
